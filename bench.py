@@ -2,7 +2,7 @@
 """bench.py -- RLHF loss hot path on B200: preference-pairs/s (DPO) and scored rollout-tokens/s (PPO) on synthetic
 batches shaped like BASELINE.json's configs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4|C5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C3|C4|C5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +23,9 @@ the path, SURVEY.md section 8d):
 prompt + generated sequence) in pinned HOST memory copied to the device inside the timed region and the metrics read
 back to the host every step.  `--impl reference` times the reference's CPU path (the oracle port of it:
 /root/reference is absent on the GPU box) on the host cores, same `config` object.
+`--dump-outputs DIR` writes what the timed path computed in its last step as DIR/<name>.npy (float32 / float64; tiles
+too large to dump whole as a fixed, seeded sample), so that two builds can be compared output for output on the same
+seeded inputs.
 """
 from __future__ import annotations
 
@@ -38,6 +41,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CONFIGS = {
@@ -75,7 +79,14 @@ def parse():
     ap.add_argument('--ctas-per-sm', type=int, default=0)
     ap.add_argument('--bwd-variant', type=int, default=-1)
     ap.add_argument('--bwd-ctas-per-sm', type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default='',
+                    help='after the timed steps, write the outputs of the last timed step as DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs dumps the outputs of --impl ours')
+    return args
 
 
 def dpo_cfg(name, args):
@@ -215,6 +226,36 @@ def peaks():
 
 
 # ---------------------------------------------------------------------------------------------------
+# --dump-outputs: host copies of the last timed step's outputs, written by main() once the run is over
+OUTPUTS = {}
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def keep_output(name, x):
+    OUTPUTS[name] = x.detach().float().cpu().numpy() if torch.is_tensor(x) else np.asarray(x, dtype=np.float64)
+
+
+def keep_tile_sample(name, tile, rows=16, elems=1 << 20):
+    """A fixed, seeded sample of a tile too large to dump whole: `rows` whole rows (last dim) and `elems` single
+    elements drawn over the whole tile."""
+    gen = torch.Generator().manual_seed(0)
+    flat = tile.detach().reshape(-1, tile.shape[-1])
+    r = torch.randperm(flat.shape[0], generator=gen)[:rows].sort().values
+    e = torch.randint(0, flat.numel(), (min(elems, flat.numel()),), generator=gen)
+    keep_output(name + '_rows', flat[r.to(flat.device)])
+    keep_output(name + '_elements', flat.reshape(-1)[e.to(flat.device)])
+
+
+def dump_outputs(path):
+    total = sum(a.nbytes for a in OUTPUTS.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit')
+    os.makedirs(path, exist_ok=True)
+    for name, a in OUTPUTS.items():
+        np.save(os.path.join(path, f'{name}.npy'), a)
+
+
+# ---------------------------------------------------------------------------------------------------
 # synthetic batches (SURVEY.md section 8d): bf16 logits ~ N(0, 2.5^2), uniform labels, left padding
 def synth_logits(n, L, V, device, seed, like=None, noise=0.3):
     out = torch.empty((n, L, V), dtype=torch.bfloat16, device=device)
@@ -257,10 +298,12 @@ def synth_preference_ids(n_pairs, L, V, pad, seed, ragged, modal=0):
 class Engine:
     """Stands in for a DeepSpeed engine whose forward has already produced the logits tile in HBM."""
 
-    def __init__(self, out_fn, leaves=()):
+    def __init__(self, out_fn, leaves=(), keep_grads=False):
         self.module = self
         self._out = out_fn
         self._leaves = leaves
+        self._keep_grads = keep_grads
+        self.last_grads = None
         self.optimizer = type('O', (), {'param_groups': [{'lr': 1e-6}]})()
 
     def __call__(self, *a, **kw):
@@ -270,6 +313,8 @@ class Engine:
         loss.backward()
 
     def step(self):
+        if self._keep_grads:  # what an optimizer step would have consumed
+            self.last_grads = [t.grad for t in self._leaves]
         for t in self._leaves:
             t.grad = None
 
@@ -290,9 +335,10 @@ def dpo_trainer_class(modality):
     return DPOTrainer
 
 
-def dpo_bench(args, c, rank, world, device, extras=True):
+def dpo_bench(args, c, rank, world, device, extras=True, dump=False):
     """One DPO config: `value` (raw launches, CUDA events), per-kernel times, `e2e` through <modality> DPOTrainer.train_step.
-    extras: also the ragged variant (dense configs) and the eager-GPU comparator."""
+    extras: also the ragged variant (dense configs) and the eager-GPU comparator.  dump: keep the outputs of the last
+    timed step of the main variant for --dump-outputs."""
     from types import SimpleNamespace
 
     from align_anything_b200 import _lib as Lb
@@ -330,6 +376,7 @@ def dpo_bench(args, c, rank, world, device, extras=True):
         stat = torch.empty((2, plan.n_rows), dtype=torch.float32, device=device)
         ev = [[torch.cuda.Event(enable_timing=True) for _ in range(5)] for _ in range(args.steps)]
         check = {}
+        last = {}
 
         def step(k=None, verify=False):
             labels = ops.strip_pad_tail(ids, lens_t, pad, strip)
@@ -341,7 +388,7 @@ def dpo_bench(args, c, rank, world, device, extras=True):
             ops._launch_fwd(ref, labels, plan, lp[1], None, None)
             if k is not None:
                 ev[k][2].record()
-            res = ops._dpo_launch(lp[0], lp[1], SCALE_COEFF, mode, ids if skip else None, True, None)  # K2: local stats
+            res = last['k2'] = ops._dpo_launch(lp[0], lp[1], SCALE_COEFF, mode, ids if skip else None, True, None)  # K2: local stats
             # N > 1: the packed metrics are all-reduced over NVLink peer memory by a one-warp kernel on a side stream,
             # so its wait for the slowest rank overlaps K1b (what DPOTrainer.train_step does)
             pending = fused.all_reduce_async(res[1], max_lanes=(7,)) if fused is not None else None
@@ -370,11 +417,17 @@ def dpo_bench(args, c, rank, world, device, extras=True):
         torch.cuda.synchronize()
         t0.record()
         for k in range(args.steps):
-            step(k)
+            stats_out = step(k)
         t1.record()
         torch.cuda.synchronize()
         barrier(world)
         clocks = sampler.stop() if (variant == main and rank == 0) else None
+        if dump and variant == main:
+            keep_output('dpo_policy_log_probs', lp[0])
+            keep_output('dpo_reference_log_probs', lp[1])
+            keep_output('dpo_per_pair', last['k2'][0])  # per pair: loss, better / worse sample reward, -, kept
+            keep_output('dpo_stats', stats_out)
+            keep_tile_sample('dpo_grad_logits', grad)
         ms = max_over_ranks(t0.elapsed_time(t1), world) / args.steps
         fwd_ms = statistics.mean((e[0].elapsed_time(e[1]) + e[1].elapsed_time(e[2])) / 2 for e in ev)
         k2_ms = statistics.mean(e[2].elapsed_time(e[3]) for e in ev)
@@ -689,9 +742,10 @@ def ppo_port_step(O, actor, refl, critic_h, rm_h, w_c, w_r, seq, prompt, pad, le
     return out
 
 
-def ppo_bench(args, rank, world, device, tail=None):
+def ppo_bench(args, rank, world, device, tail=None, dump=False):
     """BASELINE configs[3].  tail: None = the trainer's default (`PPOTrainer.tail_logits`), True / False force the
-    tail tile (actor / reference asked for the last max(R)+1 positions only, HF `logits_to_keep`) or the full tile."""
+    tail tile (actor / reference asked for the last max(R)+1 positions only, HF `logits_to_keep`) or the full tile.
+    dump: keep the outputs of the last timed step of the resident loop for --dump-outputs."""
     from types import SimpleNamespace
 
     from align_anything_b200.models.reward_model import score_model_outputs
@@ -723,19 +777,22 @@ def ppo_bench(args, rank, world, device, tail=None):
     actor_leaf = actor.requires_grad_(True)
     critic_leaf = critic_h.requires_grad_(True)
 
-    tr.actor_model = Engine(lambda: SimpleNamespace(logits=actor_leaf), (actor_leaf,))
+    tr.actor_model = Engine(lambda: SimpleNamespace(logits=actor_leaf), (actor_leaf,), keep_grads=dump)
     tr.actor_reference_model = Engine(lambda: SimpleNamespace(logits=refl))
     tr.reward_model = Engine(lambda: score_model_outputs(rm_h, w_r, None, 'last', False))
-    tr.reward_critic_model = Engine(lambda: score_model_outputs(critic_leaf, w_c, None, 'last', False), (critic_leaf, w_c))
+    tr.reward_critic_model = Engine(lambda: score_model_outputs(critic_leaf, w_c, None, 'last', False), (critic_leaf, w_c),
+                                    keep_grads=dump)
     prompt_dev = torch.empty((Bp, c['prompt_len']), dtype=torch.int64, device=device)
     seq_dev = torch.empty((Bp, L), dtype=torch.int64, device=device)
+
+    last = {}
 
     def step(e2e: bool):
         if e2e:
             prompt_dev.copy_(prompt_host, non_blocking=True)
             seq_dev.copy_(seq_host, non_blocking=True)
         moved, attn, lens = tr.postprocess_generation(prompt_dev, seq_dev)
-        inference, training = tr.score_rollout({'input_ids': moved, 'attention_mask': attn}, lens)
+        inference, training = last['training'] = tr.score_rollout({'input_ids': moved, 'attention_mask': attn}, lens)
         return tr.rl_step(inference, training), lens
 
     prompt_dev.copy_(prompt_host)
@@ -758,6 +815,17 @@ def ppo_bench(args, rank, world, device, tail=None):
         ms_dev = max_over_ranks(t0.elapsed_time(t1), world) / args.steps
         ms_wall = max_over_ranks((w1 - w0) * 1e3, world) / args.steps
         out[label] = (ms_dev, ms_wall)
+        if dump and not e2e:
+            training = last['training'][1]
+            for name in ('log_probs', 'ref_log_probs', 'reward', 'reward_values'):
+                keep_output(f'ppo_{name}', training[name])
+            for name, t in tr.last_rl_tensors.items():
+                keep_output(f'ppo_{name}', t)
+            for name, v in metrics.items():
+                keep_output('ppo_' + name.replace('/', '_'), v)
+            keep_tile_sample('ppo_grad_actor_logits', tr.actor_model.last_grads[0])
+            keep_tile_sample('ppo_grad_critic_hidden', tr.reward_critic_model.last_grads[0])
+            keep_output('ppo_grad_critic_head', tr.reward_critic_model.last_grads[1])
     eager = None
     if world == 1 and not tail and not getattr(args, 'no_eager_baseline', False):
         eager = eager_gpu_ppo(actor_leaf.detach(), refl, critic_h.detach(), rm_h, w_c.detach(), w_r, seq_dev, prompt_dev, pad, resp)
@@ -1014,8 +1082,10 @@ def main():
         v, sample = cpu_ppo_tokens_per_s(seconds, threads)
         return {'value': v, 'unit': 'tokens/s', 'cores': cpu_ppo_tokens_per_s.threads_used, 'kind': 'port', 'sample': sample}
 
+    dump = bool(args.dump_outputs) and rank == 0
+
     def run_ppo(full):
-        ppo = ppo_bench(args, rank, world, device)
+        ppo = ppo_bench(args, rank, world, device, dump=dump)
         torch.cuda.empty_cache()
         if full:
             other = ppo_bench(args, rank, world, device, tail=not ppo['config']['tail_logits'])
@@ -1036,7 +1106,7 @@ def main():
         line = run_ppo(full=True)
     else:
         c = dpo_cfg(name, args)
-        dpo = dpo_bench(args, c, rank, world, device)
+        dpo = dpo_bench(args, c, rank, world, device, dump=dump)
         line = None
         ppo = lm_head = sft = None
         others = {}
@@ -1084,6 +1154,8 @@ def main():
 
         dist.barrier()
         dist.destroy_process_group()
+    if dump:
+        dump_outputs(args.dump_outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
 

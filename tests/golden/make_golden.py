@@ -9,6 +9,8 @@ vocab 1031 to exercise the unaligned-row path; bf16 and fp32 variants).
 """
 from __future__ import annotations
 
+import gzip
+import io
 import os
 import sys
 from types import SimpleNamespace
@@ -473,19 +475,63 @@ def golden_grpo(gen):
     return out
 
 
+def golden_port_vs_reference(gen):
+    """The reference's outputs on the seeded inputs of tests/test_oracle_vs_reference.py.  The test rebuilds those
+    inputs from their seeds, so only the outputs are stored (`gen` is not used)."""
+    sys.path.insert(0, os.path.dirname(OUT))
+    import test_oracle_vs_reference as T
+
+    dpo = {}
+    for seed in range(4):
+        for dtype in (torch.bfloat16, torch.float32):
+            ids, lens, pad, pol, ref = T.dpo_inputs(seed, dtype)
+            prev = None
+            for modality in ('text', 'image', 'audio'):
+                leaf = pol.clone().requires_grad_(True)
+                tr = ref_shim.make_dpo_trainer(leaf, ref, pad, 0.1, modality)
+                res = tr.loss({'input_ids': ids, 'attention_mask': ids != pad, 'meta_info': {'response_lens': lens}})
+                res['loss'].backward()
+                grad = leaf.grad
+                if prev is not None and torch.equal(prev, grad):
+                    grad = prev  # the text and image trainers agree: one storage in the file
+                prev = grad
+                dpo[(seed, str(dtype), modality)] = dict(loss={k: v.detach() for k, v in res.items()}, grad_logits=grad)
+    ppo = {}
+    for seed in range(3):
+        ppo[seed] = []
+        for c in T.ppo_inputs(seed):
+            p = ref_shim.make_ppo_trainer(modality=c['modality'])
+            s, lp, mask, vals = c['start'], c['lp'], c['mask'], c['vals']
+            rew = p.add_kl_divergence_regularization(c['reward'], lp, c['rlp'], mask)
+            adv, ret = p.get_advantages_and_returns(vals, rew, mask, s)
+            ppo[seed].append(dict(rewards=rew, advantages=adv, returns=ret,
+                                  actor_loss=p.actor_loss_fn(c['nlp'][:, s:], lp[:, s:], adv, mask[:, s:]),
+                                  critic_loss=p.critic_loss_fn(c['nv'][:, s:], vals[:, s:], ret, mask[:, s:])))
+    return dict(dpo=dpo, ppo=ppo, layout=ref_shim.tools().move_padding_left(T.layout_inputs(), 0))
+
+
 def main():
     gen = torch.Generator().manual_seed(20260922)
     only = sys.argv[1:]
     parts = {
         'logprob': golden_logprob, 'dpo': golden_dpo, 'ppo': golden_ppo, 'ppo_step': golden_ppo_step,
         'layout': golden_layout, 'score_head': golden_score_head, 'score_head_mm': golden_score_head_mm, 'sft': golden_sft, 'grpo': golden_grpo, 'pairwise': golden_pairwise, 'saferlhf': golden_saferlhf,
+        'port_vs_reference': golden_port_vs_reference,
     }
+    compressed = {'port_vs_reference'}  # over 1 MB as a plain .pt; most of its gradient rows are zero
     for name, fn in parts.items():
         if only and name not in only:
             continue
         data = fn(gen)
         path = os.path.join(OUT, f'{name}.pt')
-        torch.save(data, path)
+        if name in compressed:
+            buf = io.BytesIO()
+            torch.save(data, buf)
+            path += '.gz'
+            with gzip.GzipFile(path, 'wb', mtime=0) as f:
+                f.write(buf.getvalue())
+        else:
+            torch.save(data, path)
         print(name, os.path.getsize(path) // 1024, 'KiB', [k for k in data])
 
 

@@ -1,6 +1,13 @@
-"""Authoring-container tests (skipped where /root/reference is absent, e.g. on the GPU box): the oracle
-port against the LIVE unmodified reference on fresh random inputs, and the in-place graft
-(`align_anything_b200.patch`) against the reference's real module tree."""
+"""The oracle port against the unmodified reference on seeded random inputs, and the in-place graft
+(`align_anything_b200.patch`) against the reference's real module tree.
+
+The port tests rebuild their inputs from the seeds below and compare bit-exactly with what the reference
+computed on them, stored in tests/golden/port_vs_reference.pt.gz (`python tests/golden/make_golden.py
+port_vs_reference` regenerates it where the reference is importable).  The graft tests import the reference's
+own packages and classes, so they run only where the reference is importable (AA_REFERENCE_ROOT)."""
+import gzip
+import io
+import os
 
 import pytest
 import torch
@@ -8,7 +15,9 @@ import torch
 from oracle import ref_port as O
 from oracle import ref_shim
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason='/root/reference not present')
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'port_vs_reference.pt.gz')
+needs_reference = pytest.mark.skipif(not ref_shim.available(),
+                                     reason='needs the reference align-anything sources (AA_REFERENCE_ROOT)')
 
 
 def _same(a, b):
@@ -16,9 +25,13 @@ def _same(a, b):
     assert torch.equal(torch.nan_to_num(a.float()), torch.nan_to_num(b.float()))
 
 
-@pytest.mark.parametrize('seed', range(4))
-@pytest.mark.parametrize('dtype', [torch.bfloat16, torch.float32])
-def test_dpo_port_vs_live_reference(seed, dtype):
+@pytest.fixture(scope='module')
+def reference_outputs():
+    with gzip.open(GOLDEN, 'rb') as f:
+        return torch.load(io.BytesIO(f.read()), weights_only=False)
+
+
+def dpo_inputs(seed, dtype):
     gen = torch.Generator().manual_seed(seed)
     V, L, B, pad = 211 + seed, 14 + seed, 2 + seed % 2, 0
     lens = torch.randint(2, L // 2, (2 * B,), generator=gen).tolist()
@@ -29,26 +42,16 @@ def test_dpo_port_vs_live_reference(seed, dtype):
         ids[0, L - 2] = pad  # interior pad
     pol = (torch.randn(2 * B, L, V, generator=gen) * 2.5).to(dtype)
     ref = (pol.float() + 0.3 * torch.randn(2 * B, L, V, generator=gen)).to(dtype)
-    for modality in ('text', 'image', 'audio'):
-        leaf = pol.clone().requires_grad_(True)
-        tr = ref_shim.make_dpo_trainer(leaf, ref, pad, 0.1, modality)
-        batch = {'input_ids': ids, 'attention_mask': ids != pad, 'meta_info': {'response_lens': lens}}
-        want = tr.loss(batch)
-        want['loss'].backward()
-        got, grad = O.dpo_forward_backward(pol, ref, ids, lens, pad, 0.1, strip=(modality != 'audio'),
-                                           skip_identical_pairs=(modality == 'audio'))
-        for k, v in want.items():
-            _same(got[k].detach(), v.detach())
-        _same(grad, leaf.grad)
+    return ids, lens, pad, pol, ref
 
 
-@pytest.mark.parametrize('seed', range(3))
-def test_ppo_port_vs_live_reference(seed):
+def ppo_inputs(seed):
+    """One dict per (dtype, value dtype, modality), in the order the reference was run."""
     gen = torch.Generator().manual_seed(100 + seed)
     B, W, start = 3, 17 + seed, 4
+    cases = []
     for dtype, vdtype in ((torch.bfloat16, torch.float32), (torch.bfloat16, torch.bfloat16), (torch.float32, torch.float32)):
         for modality in ('text', 'image', 'audio'):
-            p = ref_shim.make_ppo_trainer(modality=modality)
             lp = (-3 * torch.rand(B, W, generator=gen)).to(dtype)
             rlp = (lp.float() + 0.2 * torch.randn(B, W, generator=gen)).to(dtype)
             mask = torch.zeros(B, W, dtype=torch.bool)
@@ -56,29 +59,53 @@ def test_ppo_port_vs_live_reference(seed):
                 mask[b, 1 : start + 3 + 2 * b] = True
             reward = torch.randn(B, generator=gen)
             vals = torch.randn(B, W, generator=gen).to(vdtype)
-            hp = O.PPO_DEFAULTS
-            r1 = p.add_kl_divergence_regularization(reward, lp, rlp, mask)
-            _same(O.kl_shaped_rewards(reward, lp, rlp, mask, hp['kl_coeff'], hp['clip_range_score']), r1)
-            a1, t1 = p.get_advantages_and_returns(vals, r1, mask, start)
-            a2, t2 = O.gae_advantages_and_returns(vals, r1, mask, start, hp['gamma'], hp['gae_lambda'])
-            _same(a2, a1)
-            _same(t2, t1)
             nlp = (lp.float() + 0.3 * torch.randn(B, W, generator=gen)).to(dtype)
-            _same(O.actor_loss(nlp[:, start:], lp[:, start:], a1, mask[:, start:], hp['clip_range_ratio']),
-                  p.actor_loss_fn(nlp[:, start:], lp[:, start:], a1, mask[:, start:]))
             nv = (vals.float() + 0.5 * torch.randn(B, W, generator=gen)).to(vdtype)
-            _same(O.critic_loss(nv[:, start:], vals[:, start:], t1, mask[:, start:], hp['clip_range_value']),
-                  p.critic_loss_fn(nv[:, start:], vals[:, start:], t1, mask[:, start:]))
+            cases.append(dict(modality=modality, start=start, lp=lp, rlp=rlp, mask=mask, reward=reward, vals=vals,
+                              nlp=nlp, nv=nv))
+    return cases
 
 
-def test_layout_port_vs_live_reference():
-    t = ref_shim.tools()
+def layout_inputs():
     gen = torch.Generator().manual_seed(3)
     ids = torch.randint(0, 3, (32, 41), generator=gen)
     ids[:, :4] = 0
-    _same(O.move_padding_left(ids, 0), t.move_padding_left(ids, 0))
+    return ids
 
 
+@pytest.mark.parametrize('seed', range(4))
+@pytest.mark.parametrize('dtype', [torch.bfloat16, torch.float32])
+def test_dpo_port_vs_live_reference(seed, dtype, reference_outputs):
+    ids, lens, pad, pol, ref = dpo_inputs(seed, dtype)
+    for modality in ('text', 'image', 'audio'):
+        want = reference_outputs['dpo'][(seed, str(dtype), modality)]
+        got, grad = O.dpo_forward_backward(pol, ref, ids, lens, pad, 0.1, strip=(modality != 'audio'),
+                                           skip_identical_pairs=(modality == 'audio'))
+        for k, v in want['loss'].items():
+            _same(got[k].detach(), v)
+        _same(grad, want['grad_logits'])
+
+
+@pytest.mark.parametrize('seed', range(3))
+def test_ppo_port_vs_live_reference(seed, reference_outputs):
+    hp = O.PPO_DEFAULTS
+    for c, want in zip(ppo_inputs(seed), reference_outputs['ppo'][seed], strict=True):
+        start, lp, mask, vals = c['start'], c['lp'], c['mask'], c['vals']
+        _same(O.kl_shaped_rewards(c['reward'], lp, c['rlp'], mask, hp['kl_coeff'], hp['clip_range_score']), want['rewards'])
+        a2, t2 = O.gae_advantages_and_returns(vals, want['rewards'], mask, start, hp['gamma'], hp['gae_lambda'])
+        _same(a2, want['advantages'])
+        _same(t2, want['returns'])
+        _same(O.actor_loss(c['nlp'][:, start:], lp[:, start:], want['advantages'], mask[:, start:], hp['clip_range_ratio']),
+              want['actor_loss'])
+        _same(O.critic_loss(c['nv'][:, start:], vals[:, start:], want['returns'], mask[:, start:], hp['clip_range_value']),
+              want['critic_loss'])
+
+
+def test_layout_port_vs_live_reference(reference_outputs):
+    _same(O.move_padding_left(layout_inputs(), 0), reference_outputs['layout'])
+
+
+@needs_reference
 def test_patch_installs_on_the_reference_tree():
     """`patch.install()` rebinds the hot-path names inside the real `align_anything` package and
     `uninstall()` restores them (no kernel is launched here: CPU container)."""
@@ -136,6 +163,7 @@ def test_patch_installs_on_the_reference_tree():
     assert ref_ppo.PPOTrainer.rollout is orig_rollout
 
 
+@needs_reference
 def test_grafted_methods_find_their_helpers_on_the_reference_classes():
     """Every `self._helper(...)` a grafted method calls must exist on the patched reference class (the grafted bodies run
     on the reference's own trainer objects, which never saw our base classes)."""
@@ -172,6 +200,7 @@ def test_grafted_methods_find_their_helpers_on_the_reference_classes():
         patch.uninstall()
 
 
+@needs_reference
 @pytest.mark.parametrize('key', ['qwen2_vl', 'llava', 'qwen2_audio'])
 def test_grafted_reward_model_forward_reaches_the_real_backbones(key, golden, monkeypatch):
     """ADVICE r1 (medium): the grafted forward must reach the multimodal backbones the way the reference's own forward
