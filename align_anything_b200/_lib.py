@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get('AA_B200_LIB') or os.path.join(_HERE, 'csrc', 'libaa_b200.so')
 
 AA_BF16, AA_F16, AA_F32 = 0, 1, 2
-MODE_FAITHFUL, MODE_F32 = 0, 1
+MODE_FAITHFUL, MODE_F32, MODE_CE = 0, 1, 2  # MODE_CE: K6 / K6b only (include/aa_b200.h)
 MASK_U8, MASK_I64 = 0, 1
 STATUS_LABEL_OOB, STATUS_SHORT_SEQUENCE, STATUS_EMPTY_MASK, STATUS_DIVERGE_RANGE = 1, 2, 4, 8
 
@@ -90,6 +90,7 @@ _SIGS = {
     'aa_tail_plan_build': (c_int, [_P, c_int32, c_int32, c_int64, c_int64, c_int64, c_int32, c_int32, c_int32, c_int32, c_int32, c_int64,
                                    c_int64, _P, _P, _P]),
     'aa_tail_rows': (c_int, [_P, c_int, c_int64, _P, c_int32, c_int32, c_int32, _P, c_int64, c_int32, _P]),
+    'aa_ce_rows': (c_int, [_P, c_int32, c_int32, c_int64, c_int64, c_int64, c_int32, _P, _P, _P, _P, _P]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

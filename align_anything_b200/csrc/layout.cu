@@ -4,6 +4,8 @@
 //                        six ATen kernels in the reference.
 // aa_count_nonpad      : the per-sample `.tolist()` + remove_pad_tokens bookkeeping at
 //                        trainers/text_image_to_text/ppo.py:190-203 (a host round-trip per sample).
+// aa_ce_rows           : the valid rows of a causal-LM cross-entropy (shifted labels != ignore_index), compacted in
+//                        row order for the lm_head path that never builds the logits tile.
 #include "common.cuh"
 
 namespace aa {
@@ -212,6 +214,73 @@ __global__ void __launch_bounds__(256)
   }
 }
 
+// Stream compaction of the causal-LM cross-entropy rows in ONE block (B * L is a few ten thousand positions: a handful of
+// tiles): thread i of a tile owns ITEMS consecutive positions, a block-wide exclusive scan of the per-thread counts gives
+// each valid row its output slot, so rows come out in ascending order whatever the thread timing.
+template <int THREADS, int ITEMS>
+__global__ void __launch_bounds__(THREADS)
+    ce_rows_kernel(const int64_t *__restrict__ labels, int B, int L, int64_t sb, int64_t sl, int64_t ignore_index, int V,
+                   int64_t *__restrict__ row_index, int64_t *__restrict__ labels_out, int64_t *__restrict__ count,
+                   int32_t *status) {
+  constexpr int WARPS = THREADS / kWarp;
+  static_assert(WARPS <= kWarp, "one warp scans the warp totals");
+  __shared__ int warp_tot[WARPS];
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int64_t n = static_cast<int64_t>(B) * L;
+  int64_t carry = 0;
+  bool oob = false;
+  for (int64_t base = 0; base < n; base += static_cast<int64_t>(THREADS) * ITEMS) {
+    const int64_t p0 = base + static_cast<int64_t>(tid) * ITEMS;
+    int64_t lab[ITEMS];
+    int c = 0;
+#pragma unroll
+    for (int i = 0; i < ITEMS; ++i) {
+      const int64_t p = p0 + i;
+      lab[i] = ignore_index;
+      if (p < n) {
+        const int64_t b = p / L;
+        const int t = static_cast<int>(p - b * L);
+        if (t + 1 < L) lab[i] = labels[b * sb + static_cast<int64_t>(t + 1) * sl];  // shifted: row t predicts token t + 1
+      }
+      if (lab[i] != ignore_index) {
+        ++c;
+        oob |= (lab[i] < 0 || lab[i] >= V);
+      }
+    }
+    int x = c;  // inclusive scan inside the warp
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) warp_tot[wid] = x;
+    __syncthreads();
+    if (wid == 0) {  // inclusive scan of the warp totals
+      int w = lane < WARPS ? warp_tot[lane] : 0;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, w, o);
+        if (lane >= o) w += y;
+      }
+      if (lane < WARPS) warp_tot[lane] = w;
+    }
+    __syncthreads();
+    int64_t slot = carry + (wid > 0 ? warp_tot[wid - 1] : 0) + (x - c);
+#pragma unroll
+    for (int i = 0; i < ITEMS; ++i) {
+      if (lab[i] != ignore_index) {
+        row_index[slot] = p0 + i;
+        labels_out[slot] = lab[i];
+        ++slot;
+      }
+    }
+    carry += warp_tot[WARPS - 1];
+    __syncthreads();  // every thread has read warp_tot before the next tile overwrites it
+  }
+  if (oob && status) atomicOr(status, AA_STATUS_LABEL_OOB);
+  if (tid == 0) *count = carry;
+}
+
 }  // namespace aa
 
 using namespace aa;
@@ -276,4 +345,16 @@ extern "C" int aa_count_nonpad(const int64_t *ids, int32_t B, int32_t L, int64_t
   AA_REQUIRE(ids && counts, AA_ERR_ARG, "aa_count_nonpad: null pointer");
   count_nonpad_kernel<256><<<B, 256, 0, static_cast<cudaStream_t>(stream)>>>(ids, L, row_stride, pad_id, counts);
   return check_launch("aa_count_nonpad");
+}
+
+extern "C" int aa_ce_rows(const int64_t *labels, int32_t B, int32_t L, int64_t label_batch_stride, int64_t label_row_stride,
+                          int64_t ignore_index, int32_t V, int64_t *row_index_out, int64_t *labels_out, int64_t *count_out,
+                          int32_t *status, void *stream) {
+  AA_REQUIRE(B > 0 && L > 0 && V > 0, AA_ERR_ARG, "aa_ce_rows: bad sizes (B=%d L=%d V=%d)", B, L, V);
+  AA_REQUIRE(labels && row_index_out && labels_out && count_out, AA_ERR_ARG, "aa_ce_rows: null pointer");
+  AA_REQUIRE(row_index_out != labels_out && labels != labels_out && labels != row_index_out, AA_ERR_ARG,
+             "aa_ce_rows: aliased outputs");
+  ce_rows_kernel<1024, 4><<<1, 1024, 0, static_cast<cudaStream_t>(stream)>>>(
+      labels, B, L, label_batch_stride, label_row_stride, ignore_index, V, row_index_out, labels_out, count_out, status);
+  return check_launch("aa_ce_rows");
 }

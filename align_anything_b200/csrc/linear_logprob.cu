@@ -49,7 +49,7 @@ struct Params {
   void *out;
   int out_dtype;
   float *stat_max, *stat_logsum;
-  int faithful;
+  int faithful;  // 0: F32 (no rounding); 1: FAITHFUL (logits and log-softmax rounded to bf16); 2: CE (logits only)
   int32_t *status;
   int v_splits, tiles_per_split;  // blockIdx.y sweeps vocabulary tiles [y * tiles_per_split, ...)
   int rot_groups;                 // CTAs start their sweep (m_tile % rot_groups) * rot_step tiles into the range
@@ -57,6 +57,11 @@ struct Params {
   int group_tiles, m_tiles;       // linear block id -> (row-tile group, split, row tile in group); see the host code
   float *partial;                 // v_splits > 1: (row, split) -> {max, sum, label logit}
 };
+
+// Params::faithful of an entry point's `mode`: AA_MODE_CE rounds the logits like nn.Linear's bf16 output but keeps the
+// log-softmax (and, in K6b, p) in fp32, so that d(logits) = g * (onehot - p) is rounded once, at the bf16 store -- what
+// transformers' ForCausalLMLoss computes on `logits.float()`
+inline int rounding(int mode) { return mode == AA_MODE_FAITHFUL ? 1 : mode == AA_MODE_CE ? 2 : 0; }
 
 // d(logits) tile store of K6b: the upstream gradient per row and the padded bf16 buffer
 struct GradParams {
@@ -246,7 +251,7 @@ __global__ void __launch_bounds__(THREADS, 1)
       const float logsum = logf(s);
       float lp = (x_label - m) - logsum;
       if (label < 0 || label >= p.V) lp = __int_as_float(0x7fc00000);
-      if (p.faithful) lp = __bfloat162float(__float2bfloat16_rn(lp));
+      if (p.faithful == 1) lp = __bfloat162float(__float2bfloat16_rn(lp));
       store_from_float(p.out, row, p.out_dtype, lp);
       if (p.stat_max) p.stat_max[row] = m;
       if (p.stat_logsum) p.stat_logsum[row] = logsum;
@@ -285,7 +290,7 @@ __global__ void __launch_bounds__(THREADS, 1)
           float xs[2] = {__uint_as_float(v[j]), __uint_as_float(v[j + 1])};
           if (p.faithful) round_bf16_pair(xs[0], xs[1]);
           float ls[2] = {(xs[0] - m) - logsum, (xs[1] - m) - logsum};
-          if (p.faithful) round_bf16_pair(ls[0], ls[1]);
+          if (p.faithful == 1) round_bf16_pair(ls[0], ls[1]);
           d[j] = ex2_approx(ls[0] * kLog2e) * neg_g;  // -(p * g), every column but the label's
           d[j + 1] = ex2_approx(ls[1] * kLog2e) * neg_g;
         }
@@ -346,7 +351,7 @@ __global__ void linear_logprob_merge_kernel(const Params p) {
   const float logsum = logf(s);
   float lp = (x_label - m) - logsum;
   if (label < 0 || label >= p.V) lp = __int_as_float(0x7fc00000);
-  if (p.faithful) lp = __bfloat162float(__float2bfloat16_rn(lp));
+  if (p.faithful == 1) lp = __bfloat162float(__float2bfloat16_rn(lp));
   store_from_float(p.out, row, p.out_dtype, lp);
   if (p.stat_max) p.stat_max[row] = m;
   if (p.stat_logsum) p.stat_logsum[row] = logsum;
@@ -504,11 +509,11 @@ extern "C" int aa_linear_logprob_fwd(const void *hidden, int64_t n_rows, int32_t
                  hidden_row_stride % 8 == 0 && weight_row_stride % 8 == 0 && hidden_row_stride >= H && weight_row_stride >= H,
              AA_ERR_ALIGN, "aa_linear_logprob_fwd: operands must be 16-byte aligned with 16-byte row strides");
   AA_REQUIRE(out_dtype == AA_BF16 || out_dtype == AA_F32, AA_ERR_DTYPE, "aa_linear_logprob_fwd: out must be bf16 or f32");
-  AA_REQUIRE(mode == AA_MODE_FAITHFUL || mode == AA_MODE_F32, AA_ERR_ARG, "aa_linear_logprob_fwd: bad mode");
+  AA_REQUIRE(mode == AA_MODE_FAITHFUL || mode == AA_MODE_F32 || mode == AA_MODE_CE, AA_ERR_ARG, "aa_linear_logprob_fwd: bad mode");
   AA_REQUIRE(n_rows < (int64_t(1) << 31) - k6::BM, AA_ERR_UNSUPPORTED, "aa_linear_logprob_fwd: too many rows");
   const bool pair = k6::env().pair > 0;
   const k6::Schedule sc = k6::make_schedule(n_rows, V, pair, partial != nullptr, partial_floats);
-  k6::Params p{labels, n_rows, V, H, out, out_dtype, stat_max, stat_logsum, mode == AA_MODE_FAITHFUL ? 1 : 0, status,
+  k6::Params p{labels, n_rows, V, H, out, out_dtype, stat_max, stat_logsum, k6::rounding(mode), status,
                1, 1, k6::env().rot, k6::env().rot_step, 1, 1, partial};
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int rc = k6::launch<false>(hidden, n_rows, H, hidden_row_stride, weight, V, weight_row_stride, p,
@@ -538,12 +543,12 @@ extern "C" int aa_linear_dlogits(const void *hidden, int64_t n_rows, int32_t H, 
              AA_ERR_ALIGN, "aa_linear_dlogits: operands must be 16-byte aligned with 16-byte row strides");
   AA_REQUIRE(grad_rows_dtype == AA_BF16 || grad_rows_dtype == AA_F16 || grad_rows_dtype == AA_F32, AA_ERR_DTYPE,
              "aa_linear_dlogits: bad grad dtype");
-  AA_REQUIRE(mode == AA_MODE_FAITHFUL || mode == AA_MODE_F32, AA_ERR_ARG, "aa_linear_dlogits: bad mode");
+  AA_REQUIRE(mode == AA_MODE_FAITHFUL || mode == AA_MODE_F32 || mode == AA_MODE_CE, AA_ERR_ARG, "aa_linear_dlogits: bad mode");
   AA_REQUIRE(n_rows < (int64_t(1) << 31) - k6::BM, AA_ERR_UNSUPPORTED, "aa_linear_dlogits: too many rows");
   const bool pair = k6::env().pair > 0;
   const k6::Schedule sc = k6::make_schedule(n_rows, V, pair, true, -1);
   k6::Params p{labels, n_rows, V, H, nullptr, AA_BF16, const_cast<float *>(stat_max), const_cast<float *>(stat_logsum),
-               mode == AA_MODE_FAITHFUL ? 1 : 0, nullptr, 1, 1, 1, 1, 1, 1, nullptr};
+               k6::rounding(mode), nullptr, 1, 1, 1, 1, 1, 1, nullptr};
   k6::GradParams gp{grad_rows, grad_rows_dtype, static_cast<__nv_bfloat16 *>(dlogits), ld, k6::env().store};
   return k6::launch<true>(hidden, n_rows, H, hidden_row_stride, weight, V, weight_row_stride, p, gp, sc, pair,
                           static_cast<cudaStream_t>(stream), "aa_linear_dlogits");

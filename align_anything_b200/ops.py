@@ -24,6 +24,7 @@ __all__ = [
     'dpo_fused_loss', 'score_head', 'score_end', 'kl_rewards_and_gae', 'gae_from_rewards', 'actor_loss', 'critic_loss',
     'move_padding_left', 'count_nonpad', 'strip_pad_tail', 'ppo_pack_metrics', 'check_status', 'raise_for_status', 'status_lane', 'causal_lm_loss', 'rm_pair_loss', 'group_advantages', 'grpo_loss', 'tail_token_log_probs', 'pair_slices', 'slice_sums', 'tail_rows', 'linear_token_log_probs',
     'sequence_log_probs_from_hidden', 'fused_linear_token_log_probs', 'tail_log_probs_from_hidden', 'tail_actor_loss', 'tail_critic_loss', 'lm_head_weight',
+    'CERows', 'ce_rows', 'causal_lm_loss_from_hidden', 'causal_lm_loss_from_hidden_scaled',
 ]
 
 _REROUTE_TO_BASE = os.environ.get('AA_B200_REROUTE_BASE', '1') != '0'
@@ -521,8 +522,7 @@ class _LinearLogProbK6Fn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, hidden, weight, labels, chunk: int, mode_code: int):
-        out, stats = fused_linear_token_log_probs(hidden, weight, labels, 'faithful' if mode_code == L.MODE_FAITHFUL else 'f32',
-                                                  return_stats=True)
+        out, stats = fused_linear_token_log_probs(hidden, weight, labels, _K6_MODE_NAME[mode_code], return_stats=True)
         ctx.save_for_backward(hidden, weight, labels, stats)
         ctx.chunk, ctx.mode_code = chunk, mode_code
         return out
@@ -564,10 +564,15 @@ class _LinearLogProbK6Fn(torch.autograd.Function):
         return d_hidden, d_weight, None, None, None
 
 
+_K6_MODE_NAME = {L.MODE_FAITHFUL: 'faithful', L.MODE_F32: 'f32', L.MODE_CE: 'ce'}
+
+
 def linear_token_log_probs(hidden: torch.Tensor, weight: torch.Tensor, labels: torch.Tensor,
                            chunk_rows: int | None = None, mode: str | None = None) -> torch.Tensor:
     """gather_log_probabilities(F.linear(hidden, weight), labels) for hidden (N, H), weight (V, H), labels (N,)
-    without materialising the (N, V) logits / gradient tiles.  Differentiable in hidden and weight."""
+    without materialising the (N, V) logits / gradient tiles.  Differentiable in hidden and weight.
+    mode='ce': the rounding of a cross-entropy on `F.linear(hidden, weight).float()` -- logits rounded to the operand
+    dtype (nn.Linear's output), fp32 log-probs, d(logits) rounded once."""
     L.require_cuda(hidden, weight, labels)
     if hidden.dim() != 2 or weight.dim() != 2 or hidden.size(1) != weight.size(1) or labels.shape != hidden.shape[:1]:
         raise ValueError('expected hidden (N, H), weight (V, H), labels (N,)')
@@ -581,12 +586,12 @@ def linear_token_log_probs(hidden: torch.Tensor, weight: torch.Tensor, labels: t
         if chunk_rows is None:  # ~2 GB of d(logits) per chunk: few read-modify-write passes over the fp32 d(weight)
             chunk_rows = max(128, (2 << 30) // ((V + 255) // 256 * 256 * 2) // 128 * 128)
         return _LinearLogProbK6Fn.apply(hidden.contiguous(), weight.contiguous(), labels, int(chunk_rows),
-                                        _mode_code(mode, hidden.dtype))
+                                        L.MODE_CE if mode == 'ce' else _mode_code(mode, hidden.dtype))
     # f16 / f32 operands or H % 64 != 0: library GEMMs (cuBLAS) around K1 / K1b -- not the product's hot configuration
     if chunk_rows is None:  # ~256 MB of logits per chunk
         chunk_rows = max(128, (256 << 20) // (V * hidden.element_size()) // 128 * 128)
     return _LinearLogProbFn.apply(hidden.contiguous(), weight.contiguous(), labels, int(chunk_rows),
-                                  _mode_code(mode, hidden.dtype))
+                                  L.MODE_F32 if mode == 'ce' else _mode_code(mode, hidden.dtype))
 
 
 def fused_linear_token_log_probs(hidden: torch.Tensor, weight: torch.Tensor, labels: torch.Tensor,
@@ -601,7 +606,7 @@ def fused_linear_token_log_probs(hidden: torch.Tensor, weight: torch.Tensor, lab
     hidden, weight = _contiguous_last(hidden.detach()), _contiguous_last(weight.detach())
     labels = labels.to(torch.int64).contiguous()
     N, V = hidden.size(0), weight.size(0)
-    mode_code = _mode_code(mode, hidden.dtype)
+    mode_code = L.MODE_CE if mode == 'ce' else _mode_code(mode, hidden.dtype)
     out = torch.empty(N, dtype=torch.bfloat16 if mode_code == L.MODE_FAITHFUL else torch.float32, device=hidden.device)
     stats = torch.empty((2, max(N, 1)), dtype=torch.float32, device=hidden.device) if return_stats else None
     sc = _device_scratch(hidden.device)
@@ -1264,6 +1269,147 @@ def causal_lm_loss_scaled(logits: torch.Tensor, labels: torch.Tensor, loss_scale
     on the multiplication; log the second."""
     logits, shift = _shifted_labels(logits, labels, ignore_index)
     return _CausalLMLossFn.apply(logits, shift, int(ignore_index), float(loss_scale))
+
+
+
+# ---- the same cross-entropy from the last hidden states (fused lm_head: no logits tile) -------------------------
+class CERows:
+    """The rows a causal-LM cross-entropy scores, compacted on the device by ONE aa_ce_rows launch: flat indices
+    b * L + t of the positions whose shifted label labels[b, t + 1] != ignore_index, in ascending order, and those labels.
+
+    The lm_head kernels are sized by the number of valid rows, which only the device knows.  The count is copied into
+    pinned host memory right after the launch and an event is recorded behind the copy; n_valid() waits on that event.
+    The trainers build the plan BEFORE they enqueue the model forward (the stream is idle then: the previous step ended
+    with its host read) and read n_valid() AFTER it, so by the time the host asks, the copy finished long ago and neither
+    the host nor the device waits on the other."""
+
+    __slots__ = ('shape', 'vocab_size', 'ignore_index', '_index', '_labels', '_count', '_host', '_event', '_n')
+
+    def __init__(self, labels: torch.Tensor, vocab_size: int, ignore_index: int):
+        L.require_cuda(labels)
+        if labels.dim() != 2:
+            raise ValueError(f'expected labels (B, L), got {tuple(labels.shape)}')
+        if labels.dtype != torch.int64:
+            labels = labels.to(torch.int64)
+        B, seq = labels.shape
+        self.shape, self.vocab_size, self.ignore_index = (B, seq), int(vocab_size), int(ignore_index)
+        dev = labels.device
+        self._index = torch.empty(B * seq, dtype=torch.int64, device=dev)
+        self._labels = torch.empty(B * seq, dtype=torch.int64, device=dev)
+        self._count = torch.zeros(1, dtype=torch.int64, device=dev)
+        self._host = self._event = self._n = None
+        if B * seq == 0:
+            self._n = 0
+            return
+        L.check(L.lib().aa_ce_rows(labels.data_ptr(), B, seq, labels.stride(0), labels.stride(1), self.ignore_index,
+                                   self.vocab_size, self._index.data_ptr(), self._labels.data_ptr(), self._count.data_ptr(),
+                                   _device_scratch(dev)['status'].data_ptr(), L.stream_ptr(dev)))
+        self._start_count_copy()
+
+    def _start_count_copy(self):
+        self._host = torch.empty(1, dtype=torch.int64, pin_memory=True)
+        self._host.copy_(self._count, non_blocking=True)
+        self._event = torch.cuda.Event()
+        self._event.record(torch.cuda.current_stream(self._count.device))
+
+    def n_valid(self) -> int:
+        """The number of valid rows (host int): waits on the count copy, once."""
+        if self._n is None:
+            self._event.synchronize()
+            self._n = int(self._host[0])
+        return self._n
+
+    @property
+    def index(self) -> torch.Tensor:
+        return self._index[:self.n_valid()]
+
+    @property
+    def labels(self) -> torch.Tensor:
+        return self._labels[:self.n_valid()]
+
+
+def ce_rows(labels: torch.Tensor, vocab_size: int, ignore_index: int = -100) -> CERows:
+    """The row plan of causal_lm_loss_from_hidden for labels (B, L): one launch, an asynchronous copy of the count, no host
+    wait.  Call it before the model forward is enqueued (see CERows).  A label outside [0, vocab_size) other than
+    ignore_index sets the device status word (raise_for_status raises IndexError, as ATen's cross_entropy would)."""
+    return CERows(labels, vocab_size, ignore_index)
+
+
+class _MeanNllFn(torch.autograd.Function):
+    """loss_scale * mean(-lp) over the compact rows: ONE aa_nll_mean launch -> (loss_scale * loss, loss).  Backward: the
+    per-row upstream gradient -loss_scale * g / n_valid, which the lm_head node folds into its d(logits) pass."""
+
+    @staticmethod
+    def forward(ctx, lp, labels, ignore_index, loss_scale):
+        dev = lp.device
+        sc = _device_scratch(dev)
+        out = torch.empty(2, dtype=torch.float32, device=dev)  # [loss, -1 / n_valid]
+        partial = torch.empty(512, dtype=torch.float32, device=dev)
+        L.check(L.lib().aa_nll_mean(lp.data_ptr(), L.AA_F32, labels.data_ptr(), lp.numel(), int(ignore_index),
+                                    out[0:1].data_ptr(), out[1:2].data_ptr(), partial.data_ptr(),
+                                    sc['counter'][4:5].data_ptr(), L.stream_ptr(dev)))
+        ctx.save_for_backward(out)
+        ctx.n, ctx.loss_scale = lp.numel(), float(loss_scale)
+        loss = out[0]
+        scaled = loss if loss_scale == 1.0 else loss * float(loss_scale)
+        ctx.mark_non_differentiable(loss)
+        return scaled.clone() if scaled is loss else scaled, loss
+
+    @staticmethod
+    def backward(ctx, g, _unused):
+        (out,) = ctx.saved_tensors
+        return (out[1] * (g.float() * ctx.loss_scale)).expand(ctx.n), None, None, None
+
+
+class _NoValidRowsFn(torch.autograd.Function):
+    """Every label ignored: the loss is NaN (causal_lm_loss's 0 / 0), the gradients are zero, no lm_head work."""
+
+    @staticmethod
+    def forward(ctx, hidden, weight, loss_scale):
+        ctx.meta = (hidden.shape, hidden.dtype, weight.shape, weight.dtype, hidden.device)
+        loss = torch.full((), float('nan'), dtype=torch.float32, device=hidden.device)
+        ctx.mark_non_differentiable(loss)
+        return loss.clone(), loss
+
+    @staticmethod
+    def backward(ctx, g, _unused):
+        hs, hd, ws, wd, dev = ctx.meta
+        dh = torch.zeros(hs, dtype=hd, device=dev) if ctx.needs_input_grad[0] else None
+        dw = torch.zeros(ws, dtype=wd, device=dev) if ctx.needs_input_grad[1] else None
+        return dh, dw, None
+
+
+def causal_lm_loss_from_hidden_scaled(hidden: torch.Tensor, weight: torch.Tensor, labels: torch.Tensor, loss_scale: float,
+                                      ignore_index: int = -100, chunk_rows: int | None = None, rows: CERows | None = None):
+    """causal_lm_loss_scaled(F.linear(hidden, weight), labels, loss_scale) without the (B, L, V) logits tile or its
+    gradient -> (loss_scale * loss, loss.detach()).  hidden (B, L, H) = the model's last hidden states, weight (V, H) = its
+    bias-free lm_head (lm_head_weight), labels (B, L).  Only the valid rows are gathered (rows: the ce_rows plan, built
+    here if not given) into a compact (n_valid, H) matrix for linear_token_log_probs in the cross-entropy's rounding
+    (bf16 operands, H % 64 == 0: K6 forward, K6b + the two tcgen05 GEMMs backward; otherwise chunked library GEMMs around
+    K1 / K1b); the mean is one aa_nll_mean launch.  Differentiable in hidden and weight."""
+    L.require_cuda(hidden, weight, labels)
+    if hidden.dim() != 3 or weight.dim() != 2 or hidden.size(2) != weight.size(1) or labels.shape != hidden.shape[:2]:
+        raise ValueError(f'expected hidden (B, L, H), weight (V, H), labels (B, L); got {tuple(hidden.shape)}, '
+                         f'{tuple(weight.shape)}, {tuple(labels.shape)}')
+    if rows is None:
+        rows = ce_rows(labels, weight.size(0), ignore_index)
+    elif rows.shape != tuple(labels.shape) or rows.ignore_index != int(ignore_index) or rows.vocab_size != weight.size(0):
+        raise ValueError('the CERows plan was built for other labels, ignore_index or vocabulary')
+    n = rows.n_valid()  # the one host wait of this path; see CERows
+    if n == 0:
+        return _NoValidRowsFn.apply(hidden, weight, float(loss_scale))
+    B, seq, H = hidden.shape
+    labels_c = rows.labels
+    x = hidden.reshape(B * seq, H).index_select(0, rows.index)
+    lp = linear_token_log_probs(x, weight, labels_c, chunk_rows, mode='ce')
+    return _MeanNllFn.apply(lp, labels_c, int(ignore_index), float(loss_scale))
+
+
+def causal_lm_loss_from_hidden(hidden: torch.Tensor, weight: torch.Tensor, labels: torch.Tensor, ignore_index: int = -100,
+                               chunk_rows: int | None = None, rows: CERows | None = None) -> torch.Tensor:
+    """causal_lm_loss(F.linear(hidden, weight), labels) without the logits tile: fp32 scalar, differentiable in hidden
+    and weight (see causal_lm_loss_from_hidden_scaled)."""
+    return causal_lm_loss_from_hidden_scaled(hidden, weight, labels, 1.0, ignore_index, chunk_rows, rows)[0]
 
 
 # ---- masked mean ---------------------------------------------------------------------------------

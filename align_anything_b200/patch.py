@@ -10,7 +10,8 @@ swaps, without touching any reference file,
     get_advantages_and_returns, rl_step, ptx_step} of the text / image / audio / video trainers, and the
     multimodal trainers' actor_step (its post-generate bookkeeping); `reward_model_step` and the text trainer's
     actor_step (generate + mask) stay the reference's,
-  * SupervisedTrainer.{loss, train_step} of the text / image / audio SFT trainers (cross-entropy from K1),
+  * SupervisedTrainer.{loss, train_step} of the text / image / audio SFT trainers (cross-entropy from K1; opt-in
+    `fused_lm_head`: from the last hidden states, no logits tile),
   * GRPOTrainer.{_get_per_token_logps, train_step} and RMTrainer.{loss, train_step} of the text trainers,
   * SimPOTrainer / ORPOTrainer / KTOTrainer.{loss, train_step} (they inherit the patched DPOTrainer.compute_log_probs),
   * SafeRLHFVTrainer.{actor_step, rollout, actor_loss_fn_with_cost, add_kl_divergence_regularization_with_cost,
@@ -173,9 +174,10 @@ def install(trainers: bool = True, models: bool = True) -> dict[str, list[str]]:
                         if hasattr(src, attr):
                             _saved.append((cls, attr, cls.__dict__.get(attr, None)))
                             setattr(cls, attr, getattr(src, attr))
-            elif modname in _SFT_TARGETS:
-                _saved.append((cls, 'ignore_index', cls.__dict__.get('ignore_index', None)))
-                setattr(cls, 'ignore_index', -100)
+            elif modname in _SFT_TARGETS:  # class attributes the grafted loss reads (its helper is a module function)
+                for attr, val in (('ignore_index', -100), ('fused_lm_head', False), ('lm_head_chunk_rows', None)):
+                    _saved.append((cls, attr, cls.__dict__.get(attr, None)))
+                    setattr(cls, attr, val)
         for modname, (clsname, src) in _SLICED_TARGETS.items():
             mod = _try_import(modname)
             cls = getattr(mod, clsname, None) if mod is not None else None

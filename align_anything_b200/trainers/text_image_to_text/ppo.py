@@ -53,6 +53,9 @@ class PPOTrainer(_TextPPOTrainer):
         if self.fused_lm_head:
             out = model(**batch, output_hidden_states=True, logits_to_keep=1, **kw)
             module = getattr(model, 'module', model)
+            # lens.tolist(): the host wait of the fused path (the row gather is sized on the host; cached on the DeviceLens,
+            # so once per rollout).  Its cross-entropy sibling (ptx_step, SupervisedTrainer) waits on the valid-row count
+            # instead, copied before the forward was enqueued (ops.CERows).
             return ops.tail_log_probs_from_hidden(out.hidden_states[-1], ops.lm_head_weight(module), input_ids,
                                                   lens.tolist(), chunk_rows=self.lm_head_chunk_rows, mode=self.mode)
         logits = self._actor_logits(model, batch, lens, **kw)

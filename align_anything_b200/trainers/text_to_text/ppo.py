@@ -18,6 +18,7 @@ import torch
 
 from ... import ops
 from ...utils.multi_process import all_reduce_packed, fused_allreduce
+from .sft import causal_lm_loss_from_model
 
 __all__ = ['PPOTrainer']
 
@@ -155,9 +156,14 @@ class PPOTrainer:
 
         batch = dict(self.infer_batch(ptx_batch))
         labels = batch.pop('labels')
-        logits = self.actor_model(**batch).logits
-        # `ptx_coeff * ptx_loss` (:405): the gradient tile comes out of the single pass already multiplied
-        scaled_loss, ptx_loss = ops.causal_lm_loss_scaled(logits, labels, self.ptx_coeff)
+        out = None
+        if getattr(self, 'fused_lm_head', False):  # multimodal trainers: the lm_head on the valid rows, no logits tile
+            out = causal_lm_loss_from_model(self, self.actor_model, batch, labels, self.ptx_coeff)
+        if out is None:
+            logits = self.actor_model(**batch).logits
+            # `ptx_coeff * ptx_loss` (:405): the gradient tile comes out of the single pass already multiplied
+            out = ops.causal_lm_loss_scaled(logits, labels, self.ptx_coeff)
+        scaled_loss, ptx_loss = out
         self.actor_model.backward(scaled_loss)
         self.actor_model.step()
         ptx_loss = get_all_reduce_mean(ptx_loss.detach())

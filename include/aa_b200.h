@@ -20,7 +20,9 @@
  *   - offsets / strides are in ELEMENTS of the tensor they index;
  *   - `mode`: AA_MODE_FAITHFUL reproduces the reference's rounding points when the
  *     tensors are bf16/f16 (fp32 arithmetic, round-to-nearest-even to the tensor dtype
- *     where the reference's eager ops round); AA_MODE_F32 keeps fp32 throughout.
+ *     where the reference's eager ops round); AA_MODE_F32 keeps fp32 throughout;
+ *     AA_MODE_CE (K6 / K6b only) rounds the logits to bf16 like nn.Linear's output and keeps the
+ *     log-softmax in fp32: the rounding of transformers' ForCausalLMLoss, which upcasts the logits.
  */
 #ifndef AA_B200_H_
 #define AA_B200_H_
@@ -34,7 +36,7 @@ extern "C" {
 #define AA_B200_ABI_VERSION 3
 
 enum { AA_BF16 = 0, AA_F16 = 1, AA_F32 = 2 };
-enum { AA_MODE_FAITHFUL = 0, AA_MODE_F32 = 1 };
+enum { AA_MODE_FAITHFUL = 0, AA_MODE_F32 = 1, AA_MODE_CE = 2 };
 enum { AA_MASK_U8 = 0, AA_MASK_I64 = 1 };
 
 enum {
@@ -491,6 +493,17 @@ int aa_tail_plan_build(const int32_t *response_lens, int32_t B, int32_t seq, int
                        int64_t label_row_stride, int32_t label_tail_len, int32_t label_shift, int32_t row_shift,
                        int32_t width, int32_t copies, int64_t copy_logit_delta, int64_t copy_out_delta, int64_t *table,
                        int32_t *status, void *stream);
+
+/* The rows a causal-LM cross-entropy scores (transformers ForCausalLMLoss; trainers/text_to_text/sft.py:95-98, ppo.py:400-408),
+ * for the lm_head path that never builds the logits tile: position (b, t) of a (B, L) batch is scored against the SHIFTED
+ * label labels[b, t + 1] (the last position is ignored).  One launch writes, in ascending row order (which fixes the fp32
+ * summation order of the loss), the flat indices b * L + t of the rows whose shifted label != ignore_index into
+ * row_index_out, their labels into labels_out (both int64 [B * L] capacity) and their number into count_out[0] (int64).
+ * A label that is neither ignore_index nor in [0, V) sets AA_STATUS_LABEL_OOB (ATen's cross_entropy would raise); the row
+ * stays in the list.  Strides in elements. */
+int aa_ce_rows(const int64_t *labels, int32_t B, int32_t L, int64_t label_batch_stride, int64_t label_row_stride,
+               int64_t ignore_index, int32_t V, int64_t *row_index_out, int64_t *labels_out, int64_t *count_out,
+               int32_t *status, void *stream);
 
 /* pad_sequence([x[b][-R_b:] for b], batch_first=True) -- trainers/text_image_to_text/ppo.py:233-249 (rollout) and
  * :318-330 (rl_step: critic values), a Python loop + pad_sequence in the reference -- and its adjoint.
