@@ -2,6 +2,10 @@
 #include <stdarg.h>
 #include <stdio.h>
 
+#include <map>
+#include <mutex>
+#include <tuple>
+
 #include "common.cuh"
 
 namespace aa {
@@ -35,6 +39,22 @@ int sm_count() {
     cached_dev = dev;
   }
   return cached;
+}
+
+int resident_ctas(const void *kernel, int threads, size_t smem) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  static std::mutex mu;
+  static std::map<std::tuple<const void *, int, size_t, int>, int> cache;
+  const auto key = std::make_tuple(kernel, threads, smem, dev);
+  std::lock_guard<std::mutex> lock(mu);
+  auto it = cache.find(key);
+  if (it != cache.end()) return it->second;
+  int n = 0;
+  // a failed query leaves its error for the launch's check_launch to report; the launch then runs one CTA per SM
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, threads, smem) != cudaSuccess || n < 1) return 1;
+  cache.emplace(key, n);
+  return n;
 }
 
 }  // namespace aa

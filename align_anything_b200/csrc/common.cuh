@@ -23,6 +23,11 @@ constexpr int kWarp = 32;
 void set_error(const char *fmt, ...);
 int check_launch(const char *what);  // cudaGetLastError -> 0 or positive code (+ message)
 int sm_count();
+// CTAs of `kernel` that fit on one SM at `threads` threads and `smem` bytes of dynamic shared memory on the current
+// device (cudaOccupancyMaxActiveBlocksPerMultiprocessor, queried once per kernel, shape and device).  Persistent
+// kernels size their grid with it: a CTA beyond it waits for a resident one to retire and runs in a thinner second
+// wave.
+int resident_ctas(const void *kernel, int threads, size_t smem);
 
 #define AA_REQUIRE(cond, code, ...)     \
   do {                                  \

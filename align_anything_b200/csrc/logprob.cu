@@ -733,13 +733,29 @@ static inline int bwd_ctas() {
   return g_bwd_variant.load(std::memory_order_relaxed) >= 0 ? g_bwd_ctas_per_sm.load(std::memory_order_relaxed) : fwd_ctas();
 }
 
-// tuning: g_variant = kernel variant (units digit) + 10 * shape code:
-//   shape 0: 256 thr x 4 vec   1: 256 x 8   2: 512 x 4   3: 128 x 8   4: 256 x 2   5: 512 x 2
+// tuning: g_variant = kernel variant (units digit) + 10 * shape code.  Forward shape codes (16-bit logits):
+//   0: 128 thr x 8 vec, one CTA per row (default)   1: 256 x 8   2: 512 x 4   3: 128 x 8   4: 256 x 2   5: 512 x 2
+//   7: the launch before this layout: 128 x 8, a persistent grid of 16 CTAs/SM (9 fit), static row stride -- kept to
+//      A/B against the default in one process (bench.py --variant 70); the backward treats 7 as its default.
+// A persistent grid (codes 1-5, f32 logits, and code 0 with ctas_per_sm > 0) holds ctas_per_sm CTAs per SM, clamped
+// to the CTAs that are resident at once; 0 means all that fit.
+constexpr int kFwdLegacyShape = 7;
+
 template <typename T, int THREADS, int UNROLL>
-static int launch_fwd_shape(const FwdParams &p, int per_sm, cudaStream_t st) {
-  int64_t grid = static_cast<int64_t>(sm_count()) * per_sm;
-  if (grid > p.n_rows) grid = p.n_rows;
-  logprob_fwd_kernel<T, THREADS, UNROLL><<<static_cast<unsigned>(grid), THREADS, 0, st>>>(p);
+static int launch_fwd_shape(const FwdParams &p, int per_sm, cudaStream_t st, bool fit_resident = true) {
+  auto kern = logprob_fwd_kernel<T, THREADS, UNROLL>;
+  int64_t grid;
+  if (per_sm < 0) {
+    grid = p.n_rows < 0x7fffffff ? p.n_rows : 0x7fffffff;  // one CTA per row (the kernel strides past a full grid)
+  } else {
+    if (fit_resident) {
+      const int resident = resident_ctas(reinterpret_cast<const void *>(kern), THREADS, 0);
+      if (per_sm == 0 || per_sm > resident) per_sm = resident;
+    }
+    grid = static_cast<int64_t>(sm_count()) * per_sm;
+    if (grid > p.n_rows) grid = p.n_rows;
+  }
+  kern<<<static_cast<unsigned>(grid), THREADS, 0, st>>>(p);
   return check_launch("aa_logprob_fwd");
 }
 
@@ -757,7 +773,8 @@ static int launch_fwd_bulk(const FwdParams &p, cudaStream_t st) {
     }
     configured.store(true, std::memory_order_relaxed);
   }
-  const int per_sm = fwd_ctas() > 0 ? fwd_ctas() : 3;
+  const int resident = resident_ctas(reinterpret_cast<const void *>(kern), CONSUMERS + 32, smem);
+  const int per_sm = (fwd_ctas() > 0 && fwd_ctas() < resident) ? fwd_ctas() : resident;
   int64_t grid = static_cast<int64_t>(sm_count()) * per_sm;
   if (grid > p.n_rows) grid = p.n_rows;
   kern<<<static_cast<unsigned>(grid), CONSUMERS + 32, smem, st>>>(p);
@@ -768,21 +785,25 @@ template <typename T>
 static int launch_fwd(const FwdParams &p, cudaStream_t st) {
   if ((fwd_variant() % 10) == 1) return launch_fwd_bulk<T>(p, st);
   const int shape = (fwd_variant() / 10) % 10;
-  const int per_sm = fwd_ctas() > 0 ? fwd_ctas() : 6;
+  const int per_sm = fwd_ctas();
   if constexpr (sizeof(T) == 2) {
     switch (shape) {
       case 1: return launch_fwd_shape<T, 256, 8>(p, per_sm, st);
-      case 2: return launch_fwd_shape<T, 512, 4>(p, fwd_ctas() > 0 ? fwd_ctas() : 3, st);
-      case 3: return launch_fwd_shape<T, 128, 8>(p, fwd_ctas() > 0 ? fwd_ctas() : 12, st);
+      case 2: return launch_fwd_shape<T, 512, 4>(p, per_sm, st);
+      case 3: return launch_fwd_shape<T, 128, 8>(p, per_sm, st);
       case 4: return launch_fwd_shape<T, 256, 2>(p, per_sm, st);
-      case 5: return launch_fwd_shape<T, 512, 2>(p, fwd_ctas() > 0 ? fwd_ctas() : 3, st);
+      case 5: return launch_fwd_shape<T, 512, 2>(p, per_sm, st);
+      case kFwdLegacyShape: return launch_fwd_shape<T, 128, 8>(p, per_sm > 0 ? per_sm : 16, st, false);
       default: break;
     }
+    // default (16-bit logits): 128 threads x 8 vectors, one CTA per row.  The block scheduler starts a row's CTA
+    // whenever a resident one retires, so the rows go to whichever SM is free: a dynamic hand-out that needs no
+    // work counter and is independent of other launches on other streams.  A static split of the rows over a
+    // persistent grid finishes at the pace of the slowest SM.  Measured on the C2 tile (tools/k1_residency_ab.py,
+    // DESIGN.md §3): one CTA per row reads 6.35 TB/s, the old 16-CTAs/SM persistent grid 5.90-6.03, a resident-sized
+    // persistent grid (9 CTAs/SM) 5.82-5.85.
+    return launch_fwd_shape<T, 128, 8>(p, per_sm > 0 ? per_sm : -1, st);
   }
-  // default (16-bit logits): 128 threads x 8 vectors in flight, 16 CTAs/SM.  Measured in the sustained
-  // full-size bench (bench.py, 33.6 GB tile, SM clock ~1.75-1.85 GHz under the power cap):
-  // 128x8x16 -> 6.20 TB/s, 256x4x6 -> 5.70-5.75 TB/s; burst (tools/sweep_k1.py): 6.8 vs 6.4 TB/s.
-  if constexpr (sizeof(T) == 2) return launch_fwd_shape<T, 128, 8>(p, fwd_ctas() > 0 ? fwd_ctas() : 16, st);
   return launch_fwd_shape<T, 256, 4>(p, per_sm, st);
 }
 

@@ -605,6 +605,8 @@ static int launch_fused_shape(const FusedActorParams &p, int mode, int per_sm, F
     }
     configured.store(true, std::memory_order_relaxed);
   }
+  const int resident = resident_ctas(reinterpret_cast<const void *>(faithful ? kf : kn), CONSUMERS + 32, smem);
+  if (per_sm > resident) per_sm = resident;
   int64_t grid = static_cast<int64_t>(sm_count()) * per_sm;
   if (grid > n_work) grid = n_work;
   static const int interleave = env_int("AA_B200_FUSED_INTERLEAVE", 1);
